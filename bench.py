@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- witnesses/sec for main_proof_of_burn on B200 (BASELINE.json `metric`).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of B synthetic, valid test_pob_input.json-shaped inputs per
@@ -30,6 +30,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 for p in (ROOT, os.path.join(ROOT, "proof-of-burn_b200")):
     if p not in sys.path:
         sys.path.insert(0, p)
@@ -144,6 +145,33 @@ def shared_config(a, expr, world):
             "l2": "each step writes %.1f GB per GPU, far beyond the 126 MB L2; no flush needed" % (a.batch * 32 * n_sig / 1e9)}
 
 
+def dump_outputs(out_dir, circuit, res, n_instances=4, n_windows=16, window=4096):
+    """Write what one timed step computed, so that two builds can be compared output for output on the same inputs:
+    what the step returns (per-instance status and output signals) and a fixed sample of the witnesses it left resident
+    in HBM (the last `n_instances` of the batch, the same `n_windows` windows of `window` entries in each, drawn from a
+    fixed seed).  Every array is float64; a field element is stored as its 8 32-bit words, least significant first,
+    which float64 holds exactly.  Some 17 MB at the defaults."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+
+    def words(limbs):
+        limbs = np.asarray(limbs, dtype=np.uint64)
+        w = np.stack([limbs & np.uint64(0xFFFFFFFF), limbs >> np.uint64(32)], axis=-1)
+        return w.reshape(limbs.shape[:-1] + (2 * limbs.shape[-1],)).astype(np.float64)
+
+    n, n_sig = len(res.status), circuit.n_signals
+    window = min(window, n_sig)
+    firsts = [0, n_sig - window] + sorted(int(v) for v in np.random.default_rng(0).integers(0, n_sig - window + 1, max(0, n_windows - 2)))
+    entries = np.concatenate([np.arange(f, f + window) for f in firsts])
+    insts = list(range(max(0, n - min(n_instances, circuit.desc["n_slots"])), n))
+    sample = np.stack([np.concatenate([circuit.witness(i, f, window) for f in firsts]) for i in insts])
+    arrays = {"status": res.status.astype(np.float64), "outputs": words(res.outputs_limbs),
+              "witness_sample": words(sample), "witness_sample_entries": entries.astype(np.float64),
+              "witness_sample_instances": np.array(insts, dtype=np.float64)}
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
 def host_cores():
     try:
         return len(os.sched_getaffinity(0))
@@ -179,6 +207,8 @@ def bench_spend(a, rank, local_rank, world):
         r = c.run_packed(None, n=a.batch, staged=True, discard=True)
         dev_ms += r.timing["total_ms"]; exp_ms += r.timing["expand_ms"]; ok += r.n_ok
         launches += r.timing["expand_launches"] + r.timing["eval_launches"] + r.timing["other_launches"]
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, c, r)
     for _ in range(a.steps):
         r2 = c.run_packed(pinned.array, discard=True)
         e2e_ms += r2.timing["total_ms"]
@@ -221,7 +251,13 @@ def main():
     ap.add_argument("--reduced-batch", type=int, default=256, help="instances of the reduced (--O1-style) witness figure (0 = skip)")
     ap.add_argument("--export-sample", type=int, default=24, help="instances of the 'every witness exported to the host' figure (0 = skip)")
     ap.add_argument("--seed", type=int, default=7503)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy "
+                    "(status, output signals and a seeded sample of the resident witnesses; rank 0 only)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; the reference arm has none")
     a.warmup = max(a.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -302,6 +338,8 @@ def main():
     barrier()
     wall_ms = 1e3 * (time.time() - t_wall)
     clocks = sampler.stop(t_wall, time.time())
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, circuit, r)       # before the end-to-end arm reuses the witness slots
     # end-to-end arm (host buffers)
     for _ in range(min(a.warmup, 1)):
         step_e2e()

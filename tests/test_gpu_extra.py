@@ -113,7 +113,7 @@ def test_retain_list_materialises_only_the_named_instances():
         c.close()
 
 
-def test_rejected_instance_has_no_witness():
+def test_rejected_instance_has_no_witness(tmp_path):
     """SURVEY.md 8(b): a failed instance contributes no witness (the reference calculator aborts, tests/test.py:65-68):
     every accessor answers POB_E_REJECTED, its digest stays 0, and the neighbours are unaffected."""
     import pob_b200
@@ -121,17 +121,18 @@ def test_rejected_instance_has_no_witness():
     s = suite("test_spend")
     good, bad = s["cases"][0]["input"], s["cases"][1]["input"]
     assert s["cases"][1]["expected"] is None
+    never = str(tmp_path / "never.wtns")
     c = pob_b200.Circuit("Spend(31)", max_slots=3)
     try:
         res = c.run([good, bad, good], digest=True)
         assert res.status[0] == 0 and res.status[1] != 0 and res.status[2] == 0
         assert int(res.digests[1]) == 0 and res.digests[0] == res.digests[2] != 0
-        for call in (lambda: c.witness(1), lambda: c.witness_device_ptr(1), lambda: c.write_wtns(1, "/tmp/never.wtns"), lambda: c.selfcheck_keccak(1)):
+        for call in (lambda: c.witness(1), lambda: c.witness_device_ptr(1), lambda: c.write_wtns(1, never), lambda: c.selfcheck_keccak(1)):
             with pytest.raises(pob_b200.PobError) as e:
                 call()
             assert e.value.code == pob_b200.E_REJECTED
         import os
-        assert not os.path.exists("/tmp/never.wtns")
+        assert not os.path.exists(never)
         w = oracle.run("Spend(31)", good)
         assert np.array_equal(c.witness(2), w.limbs)
         w.free()

@@ -82,7 +82,7 @@ def test_proof_of_burn_test_shape():
         c.close()
 
 
-def test_main_proof_of_burn_shape():
+def test_main_proof_of_burn_shape(tmp_path):
     """BASELINE.json configs[1]: main_proof_of_burn = ProofOfBurn(16,4,16,50,31,2,10^19,10^20), reference fixture
     re-padded to the main shape; 215,907,954 entries (6.9 GB).  Commitment (padding-independent, so equal to the
     pinned (4,4,5) value), whole-witness digest and sampled windows vs the oracle; plus a rejected instance."""
@@ -114,7 +114,7 @@ def test_main_proof_of_burn_shape():
             wb.free()
         # a rejected main-shape instance has no witness: all three accessors refuse it, and nothing was expanded for it
         assert int(res.digests[1]) == 0
-        for call in (lambda: c.witness(1, 0, 8), lambda: c.witness_device_ptr(1), lambda: c.write_wtns(1, "/tmp/rejected_main.wtns")):
+        for call in (lambda: c.witness(1, 0, 8), lambda: c.witness_device_ptr(1), lambda: c.write_wtns(1, str(tmp_path / "rejected_main.wtns"))):
             with pytest.raises(pob_b200.PobError) as e:
                 call()
             assert e.value.code == pob_b200.E_REJECTED

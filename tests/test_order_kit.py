@@ -50,9 +50,11 @@ def test_diff_tool_verdicts(tmp_path):
 
 
 def test_order_against_real_circom_when_available():
-    """pins the witness ORDER whenever a circom binary and the reference checkout are present; otherwise states that it is unpinned"""
+    """pins the witness ORDER whenever circom is on PATH and POB_REFERENCE names a proof-of-burn checkout; otherwise states
+    that it is unpinned"""
     import diff_sym
-    ref = os.environ.get("POB_REFERENCE", "/root/reference")
-    if not shutil.which("circom") or not os.path.isdir(os.path.join(ref, "circuits")):
-        pytest.skip("circom not installed: the whole-witness ORDER remains unpinned (values, outputs, accept/reject are pinned)")
+    ref = os.environ.get("POB_REFERENCE")
+    if not shutil.which("circom") or not ref or not os.path.isdir(os.path.join(ref, "circuits")):
+        pytest.skip("needs circom on PATH and POB_REFERENCE set to a proof-of-burn checkout: the whole-witness ORDER remains "
+                    "unpinned (values, outputs, accept/reject are pinned)")
     assert diff_sym.auto(ref, ["main_spend"]) == 0
