@@ -8,6 +8,7 @@
 // k_eval on the highest-priority stream (its 32-CTA grid must get SMs while the expand grid of hundreds of thousands of
 // CTAs drains), expand on the lowest.  Slots are freed by the consumer (pob_release; stream-ordered, so the stall happens
 // on the GPU), by the built-in digest consumer, or -- only when the caller says POB_RUN_DISCARD -- at once.
+#include <cuda.h>             // driver API types only: the entry points are looked up at run time (witness slots below)
 #include <cuda_runtime.h>
 #include <fcntl.h>
 #include <unistd.h>
@@ -137,8 +138,9 @@ struct pob_handle {
     // stores (ring of RING chunks)
     static const uint32_t RING = 2;
     uint32_t chunk = 0; uint64_t store_stride = 0; uint64_t *d_stores = nullptr; uint64_t *d_inputs = nullptr;
-    // witness slots
-    std::vector<uint64_t *> slots;
+    // witness slots (slot_alloc): mapped address, and the physical allocation and mapped size behind it
+    struct SlotMem { CUmemGenericAllocationHandle handle; size_t bytes; };
+    std::vector<uint64_t *> slots; std::vector<SlotMem> slot_mem;
     std::vector<int64_t> slot_owner;              // instance (of the current / last batch) whose witness the slot holds, -1 = none
     std::vector<cudaEvent_t> slot_rel_ev; std::vector<uint8_t> slot_rel_pending;   // stream-ordered release by the consumer
     std::vector<uint32_t> last_status; uint32_t last_n = 0;
@@ -151,10 +153,12 @@ struct pob_handle {
     uint32_t xgroup = 0;                       // instances per expand launch (distinct witness slots)
     uint32_t n_round_tiles = 0;                // tiles [0, n_round_tiles) are KeccakfRound tiles, the rest code tiles
     uint64_t *d_block_base = nullptr; uint32_t n_blocks = 0;   // witness index of every KeccakfRound block (self-check)
-    // k_expand_round is launched with 85 KiB of (unused) dynamic shared memory so that only TWO of its CTAs are resident
-    // per SM: fewer concurrent write streams give the DRAM controllers longer same-row bursts -- measured 7.35 TB/s with
-    // 2 CTAs/SM vs 7.26 / 7.19 / 7.09 / 6.97 TB/s with 3 / 4 / 5 / 8, and 5.96 TB/s with 1 (profiles/r01_expand_sweep.md)
-    uint32_t round_dyn_smem = 85 * 1024;
+    // Into PLAIN slots k_expand_round is launched with 85 KiB of (unused) dynamic shared memory so that only TWO of its CTAs are
+    // resident per SM: fewer concurrent write streams give the DRAM controllers longer same-row bursts -- measured 7.35 TB/s with
+    // 2 CTAs/SM vs 7.26 / 7.19 / 7.09 / 6.97 TB/s with 3 / 4 / 5 / 8, and 5.96 TB/s with 1 (profiles/r01_expand_sweep.md).
+    // Into compressible slots the trade-off turns: 8 CTAs/SM (no cap) 1164 witnesses/s against 1108 with the 85 KiB cap
+    // (profiles/r03b_compressed_expand_sweep.log).  Set in pob_create.
+    uint32_t round_dyn_smem = 0;
     uint32_t round_threads = 256, codes_dyn_smem = 0, codes_ug = 4, codes_overlap = 0; bool serialize = false;   // changed by POB_TUNING knobs only
     int eval_threads = 512; uint32_t eval_cluster = 0, eval_prefetch = 0;   // operand prefetch measured no gain (profiles/r02c_eval_sweep.log)   // k_eval: threads per CTA; CTAs per instance (0 = chosen per launch)
     uint32_t pos_konst_bytes = 0, levels_bytes = 0, eval_smem = 0;
@@ -238,6 +242,80 @@ template <class T> static T *upload(const std::vector<T> &v) {
 static cudaEvent_t pool_event(pob_handle *h) {
     if (h->ev_used == h->ev_pool.size()) { cudaEvent_t e; CU(cudaEventCreate(&e)); h->ev_pool.push_back(e); }
     return h->ev_pool[h->ev_used++];
+}
+
+// ---- witness slots ------------------------------------------------------------------------------------------------
+// Every slot is its own cuMemCreate allocation, asked for with generic compression: the memory system then compresses each
+// line on its way from L2 to DRAM, and 97.5 % of the entries are a single bit in a 32-byte field element.  Every reader
+// (kernels, cudaMemcpy, the copy engines) still sees the plain bytes.  The driver entry points are looked up through the
+// runtime, not linked, so that the library still loads on a machine without a driver.
+namespace {
+struct DriverVmm {
+    decltype(&cuDeviceGet) device_get; decltype(&cuDeviceGetAttribute) device_attr; decltype(&cuMemGetAllocationGranularity) granularity;
+    decltype(&cuMemCreate) create; decltype(&cuMemRelease) release;
+    decltype(&cuMemAddressReserve) reserve; decltype(&cuMemAddressFree) address_free; decltype(&cuMemMap) map; decltype(&cuMemUnmap) unmap;
+    decltype(&cuMemSetAccess) set_access;
+    template <class F> static void sym(const char *name, F &fn) {
+        void *p = nullptr; cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+        if (cudaGetDriverEntryPointByVersion(name, &p, 12000, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess || !p)
+            throw std::runtime_error(std::string("the CUDA driver has no entry point ") + name);
+        fn = reinterpret_cast<F>(p);
+    }
+    DriverVmm() {
+        sym("cuDeviceGet", device_get); sym("cuDeviceGetAttribute", device_attr); sym("cuMemGetAllocationGranularity", granularity);
+        sym("cuMemCreate", create); sym("cuMemRelease", release);
+        sym("cuMemAddressReserve", reserve); sym("cuMemAddressFree", address_free); sym("cuMemMap", map); sym("cuMemUnmap", unmap);
+        sym("cuMemSetAccess", set_access);
+    }
+};
+const DriverVmm &drv() { static const DriverVmm d; return d; }
+}  // namespace
+#define CUD(call) do { CUresult r_ = (call); if (r_ != CUDA_SUCCESS) throw std::runtime_error(std::string(#call) + ": CUresult " + std::to_string((int)r_)); } while (0)
+
+static CUmemAllocationProp slot_prop(int device, bool compressible) {
+    CUmemAllocationProp p{};
+    p.type = CU_MEM_ALLOCATION_TYPE_PINNED; p.location.type = CU_MEM_LOCATION_TYPE_DEVICE; p.location.id = device;
+    p.allocFlags.compressionType = compressible ? CU_MEM_ALLOCATION_COMP_GENERIC : CU_MEM_ALLOCATION_COMP_NONE;
+    return p;
+}
+// bytes of one slot: the witness rounded up to the allocation granularity (of both props, in case a compressible create fails)
+static size_t slot_bytes(int device, uint64_t wbytes) {
+    size_t g = 1;
+    for (bool c : {true, false}) { const CUmemAllocationProp p = slot_prop(device, c); size_t gc = 0; CUD(drv().granularity(&gc, &p, CU_MEM_ALLOC_GRANULARITY_RECOMMENDED)); g = std::max(g, gc); }
+    return (size_t)((wbytes + g - 1) / g * g);
+}
+// append one slot.  The compression type is a request: granted uncompressed, the slot is plain; a compressible create that
+// fails is retried as a plain one.
+static void slot_alloc(pob_handle *h, size_t bytes, bool compressible) {
+    const DriverVmm &D = drv();
+    pob_handle::SlotMem m{0, bytes};
+    CUmemAllocationProp p = slot_prop(h->device, compressible);
+    CUresult r = D.create(&m.handle, bytes, &p, 0);
+    if (r != CUDA_SUCCESS && compressible) { p = slot_prop(h->device, false); r = D.create(&m.handle, bytes, &p, 0); }
+    if (r != CUDA_SUCCESS) throw std::runtime_error("cuMemCreate of a witness slot failed: CUresult " + std::to_string((int)r));
+    CUdeviceptr va = 0;
+    r = D.reserve(&va, bytes, 0, 0, 0);
+    if (r == CUDA_SUCCESS) {
+        r = D.map(va, bytes, 0, m.handle, 0);
+        if (r == CUDA_SUCCESS) {
+            CUmemAccessDesc ad{}; ad.location = p.location; ad.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+            r = D.set_access(va, bytes, &ad, 1);
+            if (r != CUDA_SUCCESS) D.unmap(va, bytes);
+        }
+        if (r != CUDA_SUCCESS) D.address_free(va, bytes);
+    }
+    if (r != CUDA_SUCCESS) { D.release(m.handle); throw std::runtime_error("mapping a witness slot failed: CUresult " + std::to_string((int)r)); }
+    h->slots.push_back(reinterpret_cast<uint64_t *>(va)); h->slot_mem.push_back(m);
+}
+static void slots_free(pob_handle *h) {
+    if (h->slots.empty()) return;
+    cudaDeviceSynchronize();                   // as cudaFree would: no copy or kernel of any stream may still touch a slot
+    const DriverVmm &D = drv();
+    for (size_t s = 0; s < h->slots.size(); s++) {
+        const CUdeviceptr va = reinterpret_cast<CUdeviceptr>(h->slots[s]); const size_t bytes = h->slot_mem[s].bytes;
+        D.unmap(va, bytes); D.address_free(va, bytes); D.release(h->slot_mem[s].handle);
+    }
+    h->slots.clear(); h->slot_mem.clear();
 }
 
 // ---- batch machinery ------------------------------------------------------------------------------------------
@@ -514,7 +592,7 @@ void pob_destroy(pob_handle *h) {
                     (void *)h->d_tiles, (void *)h->d_invtab, (void *)h->d_round_desc, (void *)h->d_stores, (void *)h->d_inputs, (void *)h->d_status,
                     (void *)h->d_outputs, (void *)h->d_digests, (void *)h->d_witptr, (void *)h->d_planinst, (void *)h->d_staged, (void *)h->d_prof, (void *)h->d_block_base})
         if (p) cudaFree(p);
-    for (uint64_t *s : h->slots) cudaFree(s);
+    slots_free(h);
     for (void *p : {(void *)h->h_status, (void *)h->h_outputs, (void *)h->h_digests, (void *)h->h_witptr, (void *)h->h_planinst}) if (p) cudaFreeHost(p);
     for (cudaEvent_t e : h->ev_pool) cudaEventDestroy(e);
     for (cudaEvent_t e : h->slot_rel_ev) cudaEventDestroy(e);
@@ -573,7 +651,14 @@ int pob_create(const char *main_name, const uint64_t *params, int nparams, int h
         if (const char *v = tune_env("POB_EVAL_PROFILE")) { h->prof_path = v; CU(cudaMalloc(&h->d_prof, (P.levels.size() + 3) * sizeof(long long))); }
         // witness slots: as many as fit in 80 % of free HBM after the store ring
         size_t free_b = 0, total_b = 0; CU(cudaMemGetInfo(&free_b, &total_b));
-        const uint64_t wbytes = 32ull * P.n_signals;
+        CUdevice cu_dev = 0; int compressible = 0;
+        CUD(drv().device_get(&cu_dev, device));
+        CUD(drv().device_attr(&compressible, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, cu_dev));
+        // the reduced witness measured slower into compressible slots (expand 5.41 against 6.30 TB/s, profiles/r03b_slots_ab.log)
+        if (P.opt_level) compressible = 0;
+        if (const char *v = tune_env("POB_PLAIN_SLOTS")) if (atoi(v) != 0) compressible = 0;
+        h->round_dyn_smem = compressible ? 0 : 85 * 1024;
+        const uint64_t wbytes = slot_bytes(device, 32ull * P.n_signals);
         h->store_stride = std::max<uint64_t>(32, (P.store_u64() + 31) & ~31ull);     // never 0 (constant-only gadgets such as EIP7503())
         // eval chunk: enough instances per launch to keep the SMs busy on small circuits, bounded by a ~0.5 GB store ring
         // half (main_proof_of_burn: 32; Spend: 1024)
@@ -619,7 +704,7 @@ int pob_create(const char *main_name, const uint64_t *params, int nparams, int h
         h->chunk = chunk;
         CU(cudaMalloc(&h->d_stores, (size_t)pob_handle::RING * chunk * h->store_stride * 8));
         CU(cudaMalloc(&h->d_inputs, std::max<size_t>(32, (size_t)pob_handle::RING * chunk * P.n_inputs * 32)));
-        for (uint64_t s = 0; s < nslots; s++) { uint64_t *p = nullptr; CU(cudaMalloc(&p, wbytes)); h->slots.push_back(p); }
+        for (uint64_t s = 0; s < nslots; s++) slot_alloc(h, wbytes, compressible != 0);
         if (h->eval_l2_mb) {       // tuning: keep (part of) the store ring persisting in L2 for the kernels of the eval stream
             const size_t ring = (size_t)pob_handle::RING * chunk * h->store_stride * 8, carve = (size_t)h->eval_l2_mb << 20;
             CU(cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, carve));
